@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            (N>1: launched by torch.distributed.run, one rank/GPU)
     python bench.py --impl reference ...                     (the CPU arm: the reference's algorithm on the host cores)
+    python bench.py ... --dump-outputs DIR                   (also save the last timed step's outputs, to compare builds)
 
 Workload (BASELINE.json configs[3], the configuration the metric is quoted on): synthetic 10^6-sequence x 600-column
 alignment (multiprime_b200/synth.py), k=18, degeneracy <= 256 (-n 8), <= 3 mismatches, other flags default.
@@ -55,7 +56,12 @@ def parse_args():
     ap.add_argument("--workload", default="scan", choices=["scan", "dimer"],
                     help="scan: the headline metric (default); dimer: BASELINE.json configs[4], all-pairs dimer grid")
     ap.add_argument("--primers", type=int, default=100_000, help="primers of the dimer workload")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned as DIR/<name>.npy (scan workload, --impl b200)")
+    args = ap.parse_args()
+    if args.dump_outputs and (args.workload != "scan" or args.impl != "b200"):
+        ap.error("--dump-outputs applies to the scan workload of --impl b200")
+    return args
 
 
 def host_cores() -> int:
@@ -293,6 +299,50 @@ def sharded_parity(args, rank, local, world, comm, stream):
     return out
 
 
+# columns of a row (the reference's .out TSV) that are numbers; 3 is the primer, 10 the Information column
+ROW_COLUMNS = {"position": 0, "entropy_cover": 1, "entropy_total": 2, "degenerate_number": 4, "nonsense_number": 5,
+               "coverage": 6, "mis_f_coverage": 7, "mis_r_coverage": 8, "tm": 9}
+FILTER_FLAGS = {"GC_out_of_range": 1, "di_nucleotide": 2, "hairpin": 4}
+DUMP_SAMPLE_SEQS = 1 << 14
+DUMP_SAMPLE_BYTES = 48 << 20
+
+
+def dump_outputs(out_dir, recs, app):
+    """--dump-outputs: the rows of one step, sorted by position, as one float64 array per numeric column, the primers as
+    4-bit base sets, and the Information column as GC content (-1 where the row holds only filter notes) and filter flags;
+    the per-sequence F non-cover / R non-cover / gap-row bit vectors of every row as counts over all sequences of this
+    rank and as the bits of a fixed seeded sample of sequences (the whole vectors are 375 KB per row at 10^6)"""
+    import numpy as np
+    from multiprime_b200.iupac import sets_of
+    rows = sorted((r["row"] for r in recs), key=lambda row: row[0])
+    out = {name: np.array([row[c] for row in rows], np.float64) for name, c in ROW_COLUMNS.items()}
+    out["primer_sets"] = np.array([sets_of(row[3]) for row in rows], np.float32).reshape(len(rows), K)
+    gc, flags = np.full(len(rows), -1.0), np.zeros(len(rows))
+    for i, row in enumerate(rows):
+        if not isinstance(row[10], str):
+            gc[i] = row[10]
+            continue
+        for note in row[10].split("|"):              # "GC_out_of_range (0.72)", "di_nucleotide", "hairpin"
+            flags[i] += FILTER_FLAGS[note.split(" ")[0]]
+            if note.startswith("GC_out_of_range"):
+                gc[i] = float(note.split("(")[1].rstrip(")"))
+    out["gc"], out["filter_flags"] = gc, flags
+    pos, bits = app.coverage_bits()                  # also windows whose primer the self-dimer test dropped
+    at = {p: i for i, p in enumerate(pos.tolist())}
+    bits = bits[[at[row[0]] for row in rows]]
+    n_seq = app.n_local
+    if n_seq % 32:                                   # bits past the last sequence are not part of the vectors
+        bits[:, :, -1] &= np.uint32((1 << (n_seq % 32)) - 1)
+    out["non_cover_counts"] = np.bitwise_count(bits).sum(axis=2, dtype=np.int64).astype(np.float64)
+    n_sample = min(n_seq, DUMP_SAMPLE_SEQS, DUMP_SAMPLE_BYTES // (12 * max(1, len(rows))))
+    seqs = np.sort(np.random.default_rng(0).permutation(n_seq)[:n_sample])
+    out["sample_sequences"] = seqs.astype(np.float64)
+    out["coverage_bits_sample"] = ((bits[:, :, seqs >> 5] >> (seqs & 31).astype(np.uint32)) & 1).astype(np.float32)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, arr in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), arr)
+
+
 def run_b200(args):
     from multiprime_b200 import core, synth
 
@@ -372,13 +422,16 @@ def run_b200(args):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         t0 = time.perf_counter()
-        nrows = 0
+        recs = []
         per_step = []
         for _ in range(args.steps):
             ts = time.perf_counter()
-            nrows = len(fn())
+            recs = fn()
             per_step.append(1000 * (time.perf_counter() - ts))
         e1.record()
+        nrows = len(recs)
+        if name == "value":
+            last_recs = recs
         barrier()
         wall = time.perf_counter() - t0
         ms = max(e0.elapsed_time(e1), 0.0)
@@ -404,6 +457,8 @@ def run_b200(args):
         if world > 1:
             dist.destroy_process_group()
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last_recs, app)
     ms_step = results["value"]["ms"] / args.steps
     value = evals_all / (ms_step / 1000)
     e2e_ms = results["e2e"]["ms"] / args.steps
